@@ -242,6 +242,38 @@ def run_reference(a):
 
 METRIC = "icons/sec train-step (fwd+loss+bwd) %s"
 METRIC_NAME = {"hier": "hierarchical_ordered", "fonts": "one_stage_fonts", "scaled": "scaled_hierarchical"}
+DUMP_BYTES = 60 << 20       # --dump-outputs: array data; with the .npy headers the files stay under 64 MB
+
+
+def sample_cap(sizes, budget):
+    """The largest per-array element count c with sum(min(n, c) for n in sizes) <= budget; None when all arrays fit."""
+    if sum(sizes) <= budget:
+        return None
+    left, sizes = budget, sorted(sizes)
+    for i, n in enumerate(sizes):
+        share = left // (len(sizes) - i)
+        if n > share:
+            return share
+        left -= n
+
+
+def step_results(model, out, losses, budget_bytes):
+    """{name: float32 array} of what a caller of the train step receives: the model's outputs ('out.*'), the loss terms
+    ('loss.*') and every parameter gradient ('grad.*').  When they pass `budget_bytes` in all, each array larger than a
+    common cap is replaced by a fixed seeded sample of that many of its elements (flattened, ascending index order): the
+    same shapes give the same indices, so two runs or two builds compare element for element."""
+    ts = {"out." + k: v for k, v in out.items() if torch.is_tensor(v) and v.is_floating_point()}
+    ts.update(("loss." + k, v) for k, v in losses.items() if torch.is_tensor(v))
+    ts.update(("grad." + k, p.grad) for k, p in model.named_parameters() if p.grad is not None)
+    cap = sample_cap([t.numel() for t in ts.values()], budget_bytes // 4)
+    res = {}
+    for name, t in ts.items():
+        t = t.detach()
+        if cap is not None and t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        res[name] = t.float().cpu().numpy()
+    return res
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -284,16 +316,19 @@ def run_ours(a):
     h2d = pb_h.nbytes
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
 
-    def make_step(mdl):
+    def make_step(mdl, keep=None):
         def step(c, a_, lab=None):
             mdl.zero_grad(set_to_none=True)
             out = mdl(c, a_, c, a_, label=lab, params={})
             ls = loss_fn(out, None, weights=WEIGHTS)
             ls["loss"].backward()
+            if keep is not None:
+                keep["out"], keep["losses"] = out, ls
             return ls["loss"]
         return step
 
-    step = make_step(model)
+    last = {} if a.dump_outputs else None      # the timed path's results of its latest step (for --dump-outputs)
+    step = make_step(model, last)
     cmd_in, arg_in = torch.empty_like(cmd_d), torch.empty_like(arg_d)   # device staging for the per-step H2D copies
     lab_in = torch.empty_like(lab_d) if lab_d is not None else None
 
@@ -384,8 +419,13 @@ def run_ours(a):
     if sampler:
         sampler.recording = True
     l0 = _lib.launch_count() + model.graph_kernel_launches
+    # every step draws its dropout seed from the CUDA generator, and settle() runs a timing-dependent number of steps:
+    # reseeding here makes the timed steps' masks, and so the last step's results, a function of the arguments alone
+    torch.cuda.manual_seed(1234)
     ms = timed(lambda: step(cmd_d, arg_d, lab_d), a.steps)
     launches = (_lib.launch_count() + model.graph_kernel_launches - l0) / a.steps
+    # the step's outputs live in buffers the next (CUDA-graph) step overwrites: sample them before the e2e steps run
+    dump = step_results(model, last["out"], last["losses"], DUMP_BYTES) if last is not None else None
     for _ in range(5):
         step_e2e()
     ms_e2e = timed(step_e2e, a.steps)
@@ -439,7 +479,7 @@ def run_ours(a):
         for _ in range(3):
             pstep(cmd_d, arg_d, lab_d)
         settle(pstep, pe2e, limit=20)
-        k = max(3, min(a.steps, 10))
+        k = a.steps
         pms = timed(lambda: pstep(cmd_d, arg_d, lab_d), k)
         pms_e2e = timed(pe2e, k)
         parity = {"precision": "bf16x3 (split-bf16 operands, 3 tcgen05 products per K step)", "steps": k,
@@ -548,6 +588,10 @@ def run_ours(a):
         line["cpu_baseline"] = cpu
     if ref_gpu is not None:
         line["ref_gpu"] = ref_gpu
+    if dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -622,7 +666,12 @@ def main():
     ap.add_argument("--no-parity-mode", action="store_true")
     ap.add_argument("--no-ddp-check", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's logits, losses and parameter gradients to DIR/<name>.npy (float32; "
+                         "a fixed sample of each large array; under 64 MB in all)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl == "reference":
         run_reference(a)
     else:

@@ -1,6 +1,9 @@
-"""Generates tests/golden/*.npz by EXECUTING THE REFERENCE (alexandre01/deepsvg, mounted at /root/reference).
+"""Generates tests/golden/*.npz by EXECUTING THE REFERENCE (alexandre01/deepsvg, a checkout named by $DEEPSVG_REFERENCE).
 
-Run once in the authoring container:  python tests/golden/make_golden.py
+Run once:  DEEPSVG_REFERENCE=<deepsvg checkout> python tests/golden/make_golden.py [--out DIR] [case ...]
+A case whose file would pass 1 MB is split by key into <case>.npz + <case>.part<k>.npz (tests/golden_cases.read_fixture).
+With --oracle the fp64 oracle stands in for the reference's model and loss (no checkout needed): the same inputs, weights
+and file layout, so tests/test_oracle_golden.py regenerates fixtures with it and compares them with the committed ones.
 The reference cannot travel to the GPU box, so its outputs are committed as fixtures; tests/test_oracle_golden.py
 pins oracle/svg_oracle.py against them.  Nothing from the reference is copied: it is imported, run, and only
 numbers are stored.
@@ -8,6 +11,7 @@ numbers are stored.
 Protocol (SURVEY.md 8c): the reference module is run in float64 (`.double()`), eval mode (dropout off), VAE noise injected, and the loss's aliased in-place
 `_get_padding_mask(extended=True)` replaced by its clean clone()-based equivalent ("de-aliased oracle").
 """
+import glob
 import os
 import sys
 from unittest.mock import MagicMock
@@ -18,19 +22,23 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
-for m in ["tensorboardX", "cairosvg", "IPython", "IPython.display", "moviepy", "moviepy.editor", "shapely",
-          "shapely.ops", "shapely.geometry", "matplotlib", "matplotlib.pyplot", "svgwrite"]:
-    sys.modules.setdefault(m, MagicMock())
-
-from deepsvg.model import loss as ref_loss_mod          # noqa: E402
-from deepsvg.model import utils as ref_utils            # noqa: E402
-from deepsvg.model import model as ref_model_mod        # noqa: E402
-from deepsvg.model.config import Hierarchical, HierarchicalSelfMatching, OneStageOneShot  # noqa: E402
-from deepsvg.model.loss import SVGLoss                  # noqa: E402
-from deepsvg.model.model import SVGTransformer          # noqa: E402
 
 from oracle import svg_oracle as O                      # noqa: E402
+
+
+def load_reference():
+    """Imports the reference from $DEEPSVG_REFERENCE (its optional plotting / IO dependencies mocked) and de-aliases its
+    padding mask.  Returns its modules."""
+    if not os.path.isdir(os.path.join(os.environ.get("DEEPSVG_REFERENCE", ""), "deepsvg")):
+        sys.exit("set DEEPSVG_REFERENCE to a checkout of alexandre01/deepsvg (or pass --oracle)")
+    sys.path.insert(0, os.environ["DEEPSVG_REFERENCE"])
+    for m in ["tensorboardX", "cairosvg", "IPython", "IPython.display", "moviepy", "moviepy.editor", "shapely",
+              "shapely.ops", "shapely.geometry", "matplotlib", "matplotlib.pyplot", "svgwrite"]:
+        sys.modules.setdefault(m, MagicMock())
+    from deepsvg.model import config, loss, model
+    loss._get_padding_mask = dealiased_padding_mask
+    model._get_padding_mask = dealiased_padding_mask      # perfect_matching (model.py:315) uses the same aliased add
+    return config, loss, model
 
 
 def dealiased_padding_mask(commands, seq_dim=0, extended=False):
@@ -45,9 +53,6 @@ def dealiased_padding_mask(commands, seq_dim=0, extended=False):
             return pm.unsqueeze(-1)
         return pm
 
-
-ref_loss_mod._get_padding_mask = dealiased_padding_mask
-ref_model_mod._get_padding_mask = dealiased_padding_mask      # perfect_matching (model.py:315) uses the same aliased add
 
 CASES = {
     # name: (kind, overrides, batch, store_full)
@@ -125,8 +130,9 @@ def edge_batch(cfg):
 WEIGHTS = dict(O.DEFAULT_WEIGHTS)
 
 
-def ref_cfg(kind, over):
-    c = (HierarchicalSelfMatching() if over.get("self_match") else Hierarchical()) if kind == "hierarchical" else OneStageOneShot()
+def ref_cfg(config, kind, over):
+    c = (config.HierarchicalSelfMatching() if over.get("self_match") else config.Hierarchical()) if kind == "hierarchical" \
+        else config.OneStageOneShot()
     for k, v in over.items():
         setattr(c, k, v)
     if "max_total_len" not in over:
@@ -143,12 +149,11 @@ def sample(t, n=4096):
     return f[idx]
 
 
-def run_case(name):
-    kind, over, batch, full = CASES[name]
-    cfg_o = O.make_cfg(kind, **over)
-    cfg_r = ref_cfg(kind, over)
-    params = O.make_params(cfg_o, seed=7, dtype=torch.float64)
-    model = SVGTransformer(cfg_r).double()   # fp64: no ReLU-boundary chaos between two implementations
+def run_reference(kind, over, cfg_o, params, cmd, arg, arg_dec, label, eps):
+    """The reference's SVGTransformer + SVGLoss + backward in fp64.  Returns (out, losses, grads, assignment or None)."""
+    config, loss, model_mod = load_reference()
+    cfg_r = ref_cfg(config, kind, over)
+    model = model_mod.SVGTransformer(cfg_r).double()   # fp64: no ReLU-boundary chaos between two implementations
     sd = model.state_dict()
     # the oracle's parameter inventory must be exactly the reference's parameters
     ref_param_names = {k for k, _ in model.named_parameters()}
@@ -157,25 +162,9 @@ def run_case(name):
         assert tuple(sd[k].shape) == tuple(v.shape), (k, sd[k].shape, v.shape)
     model.load_state_dict(params, strict=False)
     model.eval()
-    loss_fn = SVGLoss(cfg_r)
-    cmd, arg = edge_batch(cfg_o) if name.startswith("edge") else O.synth_batch(cfg_o, batch, seed=99)
-    assert cmd.shape[0] == batch
-    cmd, arg = cmd.double(), arg.double()
-    arg_dec = arg
-    if over.get("rel_targets"):
-        # relative-argument targets (SVGTensor.get_relative_args, difflib/tensor.py:150-168): ids in [0, 2*args_dim-2] on
-        # the slots the command uses, -1 elsewhere; drawn at random here (the model only sees them as class ids)
-        m = O.CMD_ARGS_MASK[cmd.long()].double()
-        vals = torch.randint(0, 2 * cfg_o.args_dim - 1, arg.shape, generator=torch.Generator().manual_seed(41)).double()
-        arg_dec = vals * m - (1 - m)
-    label = None
-    kw = {}
-    if cfg_o.label_condition:
-        label = torch.randint(0, cfg_o.n_labels, (batch,), generator=torch.Generator().manual_seed(5))
-        kw["label"] = label
-    eps = None
-    if cfg_o.use_vae:
-        eps = torch.randn(batch, cfg_o.dim_z, generator=torch.Generator().manual_seed(6)).double()
+    loss_fn = loss.SVGLoss(cfg_r)
+    kw = {"label": label} if label is not None else {}
+    if eps is not None:
         real = torch.randn_like
         torch.randn_like = lambda s, *a, **k: eps.reshape(s.shape).to(s.dtype)
     captured = {}
@@ -189,18 +178,49 @@ def run_case(name):
     try:
         out = model(cmd, arg, cmd, arg_dec, params={}, **kw)
     finally:
-        if cfg_o.use_vae:
+        if eps is not None:
             torch.randn_like = real
     losses = loss_fn(out, None, weights=WEIGHTS)
     model.zero_grad()
     losses["loss"].backward()
     grads = {k: (p.grad if p.grad is not None else torch.zeros_like(p)) for k, p in model.named_parameters()}
+    return out, losses, grads, captured.get("asg")
+
+
+def run_oracle(kind, over, cfg_o, params, cmd, arg, arg_dec, label, eps):
+    """oracle/svg_oracle.py in fp64 on the same inputs and weights, in place of the reference (--oracle)."""
+    out, losses, grads = O.train_step(params, cfg_o, cmd, arg, label=label, eps=eps, weights=WEIGHTS,
+                                      args_dec=arg_dec if arg_dec is not arg else None)
+    return out, losses, grads, out.get("assignment")
+
+
+def run_case(name, run_model=run_reference):
+    kind, over, batch, full = CASES[name]
+    cfg_o = O.make_cfg(kind, **over)
+    params = O.make_params(cfg_o, seed=7, dtype=torch.float64)
+    cmd, arg = edge_batch(cfg_o) if name.startswith("edge") else O.synth_batch(cfg_o, batch, seed=99)
+    assert cmd.shape[0] == batch
+    cmd, arg = cmd.double(), arg.double()
+    arg_dec = arg
+    if over.get("rel_targets"):
+        # relative-argument targets (SVGTensor.get_relative_args, difflib/tensor.py:150-168): ids in [0, 2*args_dim-2] on
+        # the slots the command uses, -1 elsewhere; drawn at random here (the model only sees them as class ids)
+        m = O.CMD_ARGS_MASK[cmd.long()].double()
+        vals = torch.randint(0, 2 * cfg_o.args_dim - 1, arg.shape, generator=torch.Generator().manual_seed(41)).double()
+        arg_dec = vals * m - (1 - m)
+    label = None
+    if cfg_o.label_condition:
+        label = torch.randint(0, cfg_o.n_labels, (batch,), generator=torch.Generator().manual_seed(5))
+    eps = None
+    if cfg_o.use_vae:
+        eps = torch.randn(batch, cfg_o.dim_z, generator=torch.Generator().manual_seed(6)).double()
+    out, losses, grads, asg = run_model(kind, over, cfg_o, params, cmd, arg, arg_dec, label, eps)
 
     fx = {"commands": cmd.float().numpy(), "args": arg.float().numpy(), "seed_params": np.int64(7)}
     if arg_dec is not arg:
         fx["args_dec"] = arg_dec.float().numpy()
-    if captured:
-        fx["assignment"] = captured["asg"].reshape(batch, -1).numpy()     # what the reference's perfect_matching picked
+    if asg is not None:
+        fx["assignment"] = asg.reshape(batch, -1).numpy()     # what the reference's perfect_matching picked
     if label is not None:
         fx["label"] = label.numpy()
     if eps is not None:
@@ -218,9 +238,29 @@ def run_case(name):
     for k, g in grads.items():
         fx["Gnorm_" + k] = np.float64(g.double().norm().item())
         fx["G_" + k] = (g if full else sample(g, 512)).detach().numpy()
-    path = os.path.join(OUT_DIR, name + ".npz")
-    np.savez_compressed(path, **fx)
-    print(name, {k: float(v) for k, v in fx.items() if k.startswith("L_")}, os.path.getsize(path) // 1024, "KB")
+    kb = save_fixture(OUT_DIR, name, fx) // 1024
+    print(name, {k: float(v) for k, v in fx.items() if k.startswith("L_")}, kb, "KB")
+
+
+MAX_FILE_BYTES = 1 << 20
+
+
+def save_fixture(out_dir, name, fx):
+    """Writes `fx` as out_dir/name.npz, split by key into name.npz, name.part1.npz, ... when one file would pass
+    MAX_FILE_BYTES (compressed).  Returns the total size in bytes."""
+    for p in glob.glob(os.path.join(out_dir, name + ".part*.npz")):
+        os.remove(p)
+    keys = list(fx)
+    for n in range(1, len(keys) + 1):
+        paths = [os.path.join(out_dir, name + (".npz" if i == 0 else ".part%d.npz" % i)) for i in range(n)]
+        for path, chunk in zip(paths, np.array_split(np.array(keys, dtype=object), n)):
+            np.savez_compressed(path, **{k: fx[k] for k in chunk})
+        sizes = [os.path.getsize(p) for p in paths]
+        if max(sizes) <= MAX_FILE_BYTES:
+            return sum(sizes)
+        for p in paths[1:]:
+            os.remove(p)
+    raise RuntimeError("%s: a single array passes %d bytes" % (name, MAX_FILE_BYTES))
 
 
 OUT_DIR = HERE
@@ -232,5 +272,9 @@ if __name__ == "__main__":
         OUT_DIR = argv[argv.index("--out") + 1]
         del argv[argv.index("--out"):argv.index("--out") + 2]
         os.makedirs(OUT_DIR, exist_ok=True)
+    runner = run_reference
+    if "--oracle" in argv:
+        argv.remove("--oracle")
+        runner = run_oracle
     for n in (argv or CASES):
-        run_case(n)
+        run_case(n, runner)

@@ -1,6 +1,6 @@
 """Generates tests/golden/pack_batch.npz by EXECUTING the reference's batch assembly
 (SVGTensorDataset.get_data, svgtensor_dataset.py:164-205, with SVGTensor.add_eos/add_sos/pad, difflib/tensor.py:108-143)
-on random raw path tensors.  Run once in the authoring container: python tests/golden/make_pack_golden.py
+on random raw path tensors.  Run once: DEEPSVG_REFERENCE=<deepsvg checkout> python tests/golden/make_pack_golden.py
 Only numbers are stored; tests/test_pack.py checks deepsvg_b200.pack_icons (native packer) against them.
 """
 import os
@@ -12,7 +12,9 @@ import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, "/root/reference")
+if not os.path.isdir(os.path.join(os.environ.get("DEEPSVG_REFERENCE", ""), "deepsvg")):
+    sys.exit("set DEEPSVG_REFERENCE to a checkout of alexandre01/deepsvg")
+sys.path.insert(0, os.environ["DEEPSVG_REFERENCE"])
 for m in ["tensorboardX", "cairosvg", "IPython", "IPython.display", "moviepy", "moviepy.editor", "shapely",
           "shapely.ops", "shapely.geometry", "matplotlib", "matplotlib.pyplot", "svgwrite", "pandas", "PIL", "PIL.Image",
           "networkx", "sklearn", "sklearn.cluster", "bs4", "numpy.core.multiarray"]:

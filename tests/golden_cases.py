@@ -1,5 +1,6 @@
 """The fixture cases of tests/golden/make_golden.py, restated so the tests do not import the generator
-(which needs /root/reference)."""
+(which needs a checkout of the original deepsvg)."""
+import glob
 import os
 
 import numpy as np
@@ -45,8 +46,17 @@ CASES = {
 }
 
 
+def read_fixture(directory, name):
+    """The arrays of fixture `name`: directory/name.npz plus the name.part<k>.npz files of a case that
+    make_golden.py split to keep every file under 1 MB."""
+    fx = {}
+    for p in [os.path.join(directory, name + ".npz")] + sorted(glob.glob(os.path.join(directory, name + ".part*.npz"))):
+        fx.update(np.load(p, allow_pickle=False))
+    return fx
+
+
 def load_case(name):
     kind, over, full = CASES[name]
     cfg = O.make_cfg(kind, **over)
-    fx = dict(np.load(os.path.join(HERE, "golden", name + ".npz"), allow_pickle=False))
+    fx = read_fixture(os.path.join(HERE, "golden"), name)
     return cfg, fx, full

@@ -6,7 +6,7 @@ import pytest
 import torch
 
 from oracle import svg_oracle as O
-from tests.golden_cases import CASES, load_case
+from tests.golden_cases import CASES, load_case, read_fixture
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -89,19 +89,20 @@ def test_matmul_modes_are_close():
     assert e3 < 2e-4 and e3 < e1 / 20, (e3, e1)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/deepsvg"), reason="the reference checkout exists only in the authoring container")
 def test_fixtures_regenerate_from_the_reference(tmp_path):
-    """Re-executes the reference (tests/golden/make_golden.py) and requires the committed fixtures to come out again
-    (inputs bit for bit; fp64 results to 1e-10 relative, so a different BLAS thread split cannot make it flaky)."""
+    """Re-runs the fixture generator (tests/golden/make_golden.py) with the fp64 oracle standing in for the reference's
+    model and loss, and requires the committed fixtures -- the reference's own results -- to come out again: inputs,
+    weights and key set bit for bit, fp64 results to 1e-10 relative (a different BLAS thread split cannot make it flaky).
+    Run the generator without --oracle on a checkout of the reference to regenerate the fixtures themselves."""
     import subprocess
     import sys
-    names = ["tiny_hier", "edge_hier"]
-    r = subprocess.run([sys.executable, os.path.join(HERE, "golden", "make_golden.py"), "--out", str(tmp_path)] + names,
-                       capture_output=True, text=True, timeout=600)
+    names = ["tiny_hier", "edge_hier", "tiny_hier_vae_label", "tiny_one_stage", "tiny_selfmatch", "tiny_sketchformer"]
+    r = subprocess.run([sys.executable, os.path.join(HERE, "golden", "make_golden.py"), "--oracle", "--out", str(tmp_path)]
+                       + names, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     for n in names:
-        new = dict(np.load(os.path.join(str(tmp_path), n + ".npz"), allow_pickle=False))
-        old = dict(np.load(os.path.join(HERE, "golden", n + ".npz"), allow_pickle=False))
+        new = read_fixture(str(tmp_path), n)
+        old = read_fixture(os.path.join(HERE, "golden"), n)
         assert sorted(new) == sorted(old), n
         for k in old:
             if old[k].dtype.kind == "f" and not k.startswith(("commands", "args")):
